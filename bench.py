@@ -8,7 +8,7 @@ NORMAL_PHASE|MINTIME} on BASELINE config 2 (office.pcd 200x120x40 @0.1 m, B = 10
 collective; scaling = weak), value = replans of all ranks / max-over-ranks device time.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                  [--evals 64] [--batch 1024] [--no-esdf512]
+                  [--evals 64] [--batch 1024] [--no-esdf512] [--dump-outputs DIR]
 
 --impl reference times the CPU restatement of the reference (oracle/, all host threads)
 on the same workload; the unmodified reference cannot be built here (ROS1/Eigen3/PCL/NLopt
@@ -391,7 +391,7 @@ class GpuPlanner:
         m.pin(self.x_host)
         self._tcs_view = np.frombuffer(self.tcs, dtype=np.uint8)
         m.pin(self._tcs_view)
-        self.n_clusters = 0
+        self.clusters, self.n_clusters = [], 0
         # result buffers of the optimiser, reused every replan (the reference keeps best_variable_ as a member)
         self.opt_out = (np.empty_like(self.x_host), np.empty(batch, dtype=np.float64), np.empty(batch, dtype=np.int32))
         # the frontier subsystem has its own stream in the library: the search is enqueued first
@@ -407,6 +407,10 @@ class GpuPlanner:
         self.ff.reset_flags()
         self.ff.search_box_begin(self.g.origin, self.g.map_max)
 
+    def _frontier_end(self):
+        self.clusters = self.ff.search_box_end()
+        self.n_clusters = len(self.clusters)
+
     def l2_flush(self):
         self.flush.zero_()
 
@@ -416,7 +420,7 @@ class GpuPlanner:
         if not (self.overlap and self.solver_first):
             self._frontier_begin()
         if not self.overlap:
-            self.n_clusters = len(self.ff.search_box_end())
+            self._frontier_end()
         self.m.updateESDF3d()
         h = self.m.handle
         # the solver loop of BsplineOptimizer::optimize() on the device: K = max_eval cost/gradient
@@ -431,7 +435,7 @@ class GpuPlanner:
         if self.overlap:
             if self.solver_first:
                 self._frontier_begin()
-            self.n_clusters = len(self.ff.search_box_end())
+            self._frontier_end()
 
     def replan_e2e(self):
         """Through the reference-facing host API with HOST buffers: occupancy H2D, ESDF update,
@@ -461,6 +465,38 @@ class GpuPlanner:
                                               out=self.opt_out, exact_evals=True)
         self.last_neval = ne
         return out, f
+
+    def dump_outputs(self, out_dir, max_traj=32768):
+        """What the last resident replan handed back -- the ESDF, the frontier clusters, and the solver's best
+        variables, costs and evaluation counts -- as out_dir/<name>.npy in float32 / float64 (integers are exact in
+        float64), about 4.5 MB at the default batch.  Above max_traj trajectories the solver's outputs are a fixed
+        seeded sample of them (traj_index), which keeps the whole dump under 64 MB."""
+        os.makedirs(out_dir, exist_ok=True)
+        self.torch.cuda.synchronize(self.dev)
+        cl = self.clusters
+        rows = np.arange(self.B)
+        if self.B > max_traj:
+            rows = np.sort(np.random.default_rng(0).choice(self.B, max_traj, replace=False))
+
+        def cat(arrays, empty_shape):
+            return np.concatenate(arrays).astype(np.float64) if arrays else np.zeros(empty_shape)
+
+        out = {
+            "esdf": self.m.download(dtype=np.float32),                                     # [nx, ny, nz] metres
+            "traj_index": rows.astype(np.float64),
+            "x_best": self.d_xw.cpu().numpy()[rows],                                       # [B, 3 * 20 + 1]
+            "f_best": self.d_f.cpu().numpy()[rows],                                        # [B]
+            "n_eval": self.d_n.cpu().numpy()[rows].astype(np.float64),                     # [B]
+            "frontier_cell_offsets": np.cumsum([0] + [c.cells_addr_.size for c in cl]).astype(np.float64),
+            "frontier_cells": cat([c.cells_addr_ for c in cl], (0,)),                       # voxel addresses, BFS order
+            "frontier_filtered_offsets": np.cumsum([0] + [len(c.filtered_cells_) for c in cl]).astype(np.float64),
+            "frontier_filtered": cat([np.reshape(c.filtered_cells_, (-1, 3)) for c in cl], (0, 3)),
+            "frontier_average": cat([np.reshape(c.average_, (1, 3)) for c in cl], (0, 3)),
+            "frontier_box_min": cat([np.reshape(c.box_min_, (1, 3)) for c in cl], (0, 3)),
+            "frontier_box_max": cat([np.reshape(c.box_max_, (1, 3)) for c in cl], (0, 3)),
+        }
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v)
 
     def e2e_bytes(self):
         nv = self.g.nvox
@@ -877,6 +913,8 @@ def run_ours(args):
     if evals_min != args.evals:
         raise SystemExit("bench.py: the solver stopped after %d < %d evaluations on some trajectory -- the unit of work "
                          "of the metric (B x K combineCost) was not performed" % (evals_min, args.evals))
+    if args.dump_outputs and rank == 0:
+        P.dump_outputs(args.dump_outputs)
     tt = torch.tensor([dev_ms], dtype=torch.float64, device="cuda:%d" % local)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -913,7 +951,7 @@ def run_ours(args):
         except Exception as e:  # noqa: BLE001
             sharded = {"error": repr(e)}
 
-    config5 = None if args.no_config5 else config5_arm(local, rank, world, args)
+    config5 = None if args.no_config5 else config5_arm(local, rank, world, args, steps=args.steps)
 
     if rank != 0:
         if world > 1:
@@ -1026,6 +1064,8 @@ def main():
     ap.add_argument("--no-sharded", action="store_true", help="skip the config-4 z-sharded ESDF arm at N > 1")
     ap.add_argument("--no-config5", action="store_true", help="skip the office3 / 4096-trajectory replan (BASELINE config 5)")
     ap.add_argument("--no-overlap", action="store_true", help="run the frontier search after the ESDF update instead of beside it")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last resident replan "
+                    "computed (ESDF, frontier clusters, solver results) to DIR/<name>.npy; rank 0 only")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

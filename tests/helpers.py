@@ -31,6 +31,21 @@ def make_sdf_map(fuel, g, inflate, tri, optimistic=False, signed=False):
     return m
 
 
+def sdf_map_geometry(params):
+    """map_voxel_num_, map_origin_ and map_size_ as the reference's SDFMap::initMap derives them from its
+    sdf_map/* parameters (sdf_map.cpp:33-37): the map is centred in x, y and starts at ground_height in z"""
+    size = np.array([params["map_size_" + a] for a in "xyz"])
+    n = tuple(int(np.ceil(s / params["resolution"])) for s in size)
+    return n, np.array([-size[0] / 2.0, -size[1] / 2.0, params["ground_height"]]), size
+
+
+def viewpoint_rows(visib, yaw, pos):
+    """the viewpoints of one cluster as sorted rows (-visib, yaw, x, y, z): the reference sorts them by visib_num_
+    with std::sort, whose order among ties is unspecified, so they are compared as multisets"""
+    rows = np.column_stack([-np.asarray(visib, np.float64), yaw, np.reshape(pos, (-1, 3))])
+    return rows[np.lexsort(rows.T[::-1])]
+
+
 def orc_grid(orc, g):
     return orc.make_grid(g.n, g.res, g.origin, g.box_min, g.box_max)
 

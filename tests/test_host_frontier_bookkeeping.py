@@ -3,16 +3,18 @@ computeFrontiersToVisit / isFrontierCovered around the device calls) against the
 frontier_finder.cpp over a multi-frame exploration episode.  The device calls of the mirror are replaced by the oracle
 here (no GPU needed), so what is compared is exactly the host logic: which stored clusters are removed when the map
 changes (haveOverlap + isFrontierChanged), removed_ids_, the dormant list, id assignment, viewpoint filtering / order.
-Skipped where oracle/_ref was not built (no /root/reference)."""
+The reference's side of the episode, ref_episode(), is recorded by tools/make_ref_pins.py into
+tests/golden/ref_pins.npz (tests/ref_pins.py); the test compares the mirror with those stored lists."""
 import numpy as np
-import pytest
 
 import oracle as O
 from fuel_b200 import workloads as W
 from fuel_b200.frontier_finder import Frontier, FrontierFinder
+from tests import ref_pins as RP
+from tests.helpers import sdf_map_geometry, viewpoint_rows
 
 O.build()
-pytestmark = pytest.mark.skipif(O.ref_raycast() is None, reason="oracle/_ref/libfuel_ref.so not built (no /root/reference)")
+MODULE = "test_host_frontier_bookkeeping"
 
 MAP = dict(resolution=0.1, map_size_x=8.0, map_size_y=6.0, map_size_z=3.0, ground_height=-0.5, obstacles_inflation=0.199,
            local_bound_inflate=0.5, local_map_margin=50, default_dist=0.0, optimistic=0, signed_dist=0, p_hit=0.65, p_miss=0.35,
@@ -31,8 +33,8 @@ def logit(p):
 class FakeMap:
     """what the mirror needs from SDFMap, without a device"""
 
-    def __init__(self, ref):
-        self.shape, self.resolution_, self.map_origin_ = ref.n, ref.res, ref.origin
+    def __init__(self, n, res, origin):
+        self.shape, self.resolution_, self.map_origin_ = n, res, origin
         self.handle = None
         self.update_min_, self.update_max_ = np.zeros(3), np.zeros(3)
 
@@ -70,64 +72,105 @@ class OracleBackedFinder(FrontierFinder):
         return np.stack([o["pos"] for o in out]), np.stack([o["yaw"] for o in out]), np.stack([o["visib"] for o in out])
 
 
-def same_lists(mine, theirs):
-    assert len(mine) == len(theirs)
-    for a, b in zip(mine, theirs):
-        assert np.array_equal(a.cells_addr_, b["addr"])
-        assert np.array_equal(a.average_, b["average"])
+def list_arrays(prefix, addrs, averages):
+    """a frontier list as flat arrays: cells (BFS order) and averages"""
+    return {prefix + "offsets": np.cumsum([0] + [len(a) for a in addrs]),
+            prefix + "addr": np.concatenate(addrs) if addrs else np.zeros(0, np.int64),
+            prefix + "average": np.reshape(averages, (-1, 3))}
+
+
+def mirror_arrays(prefix, ftrs):
+    return list_arrays(prefix, [f.cells_addr_ for f in ftrs], [f.average_ for f in ftrs])
+
+
+def ref_arrays(prefix, ftrs):
+    return list_arrays(prefix, [f["addr"] for f in ftrs], [f["average"] for f in ftrs])
+
+
+# the robot reveals one ball of space per frame, moving through the room
+PATH = [(18, 20, 12), (28, 24, 12), (38, 30, 13), (48, 32, 12), (58, 36, 12), (60, 22, 12), (46, 16, 12), (30, 40, 14)]
+BOX = ((-3.6, -2.6, -0.3), (3.6, 2.6, 2.2))
+
+
+class Episode:
+    """the map state of the episode: tri-state and known inflation, updated in place frame by frame"""
+
+    def __init__(self):
+        self.n, self.origin, _ = sdf_map_geometry(MAP)
+        rng = np.random.default_rng(12)
+        self.inflate = (rng.random(self.n) < 0.003).astype(np.int8)
+        self.XYZ = np.meshgrid(*[np.arange(k) for k in self.n], indexing="ij")
+        self.tri = np.full(self.n, W.UNKNOWN, np.uint8)
+        self.inf_known = np.zeros(self.n, np.int8)
+
+    def reveal(self, k, c):
+        """-> the newly known voxels and the updated box of frame k"""
+        X, Y, Z = self.XYZ
+        ball = ((X - c[0]) ** 2 + (Y - c[1]) ** 2 + 3.0 * (Z - c[2]) ** 2) < (11 + (k % 3)) ** 2
+        newly = ball & (self.tri == W.UNKNOWN)
+        self.tri[newly] = np.where(self.inflate[newly] == 1, W.OCCUPIED, W.FREE)
+        self.inf_known[newly] = self.inflate[newly]
+        idx = np.argwhere(newly)
+        assert len(idx)
+        res = MAP["resolution"]
+        return newly, self.origin + idx.min(axis=0) * res, self.origin + (idx.max(axis=0) + 1) * res
+
+
+def ref_episode():
+    ref = O.RefSDFMap(**MAP)
+    ep = Episode()
+    ref.inflate[:] = 0
+    ref.occupancy[:] = logit(0.12) - 0.01
+    rff = O.RefFrontierFinder(ref, PU, **FF)
+    occ = ref.occupancy.reshape(ref.n)
+    out = {}
+    for k, c in enumerate(PATH):
+        newly, umin, umax = ep.reveal(k, c)
+        occ[newly] = np.where(ep.inflate[newly] == 1, logit(0.90), logit(0.12))
+        ref.inflate[:] = ep.inf_known.reshape(-1)
+        ref.R.ref_map_set_updated_box(ref.h, O._p(umin), O._p(umax))
+        # searchFrontiers(); computeFrontiersToVisit()
+        out.update(ref_arrays("f%d_tmp_" % k, rff.search_frontiers()))
+        out["f%d_removed" % k] = np.asarray(rff.removed_ids(), np.int64)
+        out["f%d_flags" % k] = rff.flags.copy()
+        visit, dormant = rff.compute_to_visit()
+        out.update(ref_arrays("f%d_visit_" % k, visit))
+        out.update(ref_arrays("f%d_dormant_" % k, dormant))
+        out["f%d_ids" % k] = [v["id"] for v in visit]
+        for i, v in enumerate(visit):
+            out["f%d_vp%d" % (k, i)] = viewpoint_rows(v["view_visib"], v["view_yaw"], v["view_pos"])
+    rff.close()
+    ref.close()
+    return out
 
 
 def test_exploration_episode_matches_reference():
-    ref = O.RefSDFMap(**MAP)
-    n = ref.n
-    rng = np.random.default_rng(12)
-    inflate = (rng.random(n) < 0.003).astype(np.int8)
-    X, Y, Z = np.meshgrid(*[np.arange(k) for k in n], indexing="ij")
-    tri = np.full(n, W.UNKNOWN, np.uint8)
-    ref.inflate[:] = 0
-    ref.occupancy[:] = logit(0.12) - 0.01
-    g = ref.grid((-3.6, -2.6, -0.3), (3.6, 2.6, 2.2))
-    rff = O.RefFrontierFinder(ref, PU, **FF)
-    fmap = FakeMap(ref)
-    inf_known = np.zeros(n, np.int8)
-    mine = OracleBackedFinder(fmap, g, tri, inf_known, **FF)
+    P = RP.load(MODULE, "episode", REF_PINS)
+    ep = Episode()
+    g = O.make_grid(ep.n, MAP["resolution"], ep.origin, BOX[0], BOX[1], map_size=sdf_map_geometry(MAP)[2])
+    fmap = FakeMap(ep.n, MAP["resolution"], ep.origin)
+    mine = OracleBackedFinder(fmap, g, ep.tri, ep.inf_known, **FF)
     mine.setViewParams(min_visib_num=FF["min_visib_num"], min_view_finish_fraction=FF["min_view_finish_fraction"])
-    occ = ref.occupancy.reshape(n)
     total_removed = 0
-    # the robot reveals one ball of space per frame, moving through the room
-    path = [(18, 20, 12), (28, 24, 12), (38, 30, 13), (48, 32, 12), (58, 36, 12), (60, 22, 12), (46, 16, 12), (30, 40, 14)]
-    for k, c in enumerate(path):
-        ball = ((X - c[0]) ** 2 + (Y - c[1]) ** 2 + 3.0 * (Z - c[2]) ** 2) < (11 + (k % 3)) ** 2
-        newly = ball & (tri == W.UNKNOWN)
-        tri[newly] = np.where(inflate[newly] == 1, W.OCCUPIED, W.FREE)
-        occ[newly] = np.where(inflate[newly] == 1, logit(0.90), logit(0.12))
-        inf_known[newly] = inflate[newly]
-        ref.inflate[:] = inf_known.reshape(-1)
-        idx = np.argwhere(newly)
-        assert len(idx)
-        umin = ref.origin + idx.min(axis=0) * ref.res
-        umax = ref.origin + (idx.max(axis=0) + 1) * ref.res
-        ref.R.ref_map_set_updated_box(ref.h, O._p(umin), O._p(umax))
-        fmap.update_min_, fmap.update_max_ = umin, umax
-        # reference: searchFrontiers(); computeFrontiersToVisit()   |   mirror: the same two calls
-        tmp_ref = rff.search_frontiers()
+    for k, c in enumerate(PATH):
+        _, fmap.update_min_, fmap.update_max_ = ep.reveal(k, c)
         mine.searchFrontiers()
-        assert mine.removed_ids_ == rff.removed_ids(), "frame %d removed_ids_" % k
+        for key, v in mirror_arrays("f%d_tmp_" % k, mine.tmp_frontiers_).items():
+            P.check(key, v)
+        P.check("f%d_removed" % k, np.asarray(mine.removed_ids_, np.int64), "removed_ids_")
         total_removed += len(mine.removed_ids_)
-        same_lists(mine.tmp_frontiers_, tmp_ref)
-        assert np.array_equal(mine.flag.reshape(-1), rff.flags), "frame %d flags" % k
-        visit_ref, dormant_ref = rff.compute_to_visit()
+        P.check("f%d_flags" % k, mine.flag.reshape(-1), "frontier_flag_")
         mine.computeFrontiersToVisit()
-        same_lists(mine.frontiers_, visit_ref)
-        same_lists(mine.dormant_frontiers_, dormant_ref)
-        for a, b in zip(mine.frontiers_, visit_ref):
-            assert a.id_ == b["id"]
-            va = sorted((-v[2], v[1], tuple(v[0])) for v in a.viewpoints_)
-            vb = sorted(zip(-b["view_visib"], b["view_yaw"], map(tuple, b["view_pos"])))
-            assert len(va) == len(vb)
-            for p, q in zip(va, vb):
-                assert p[0] == q[0] and p[2] == q[2] and (p[1] == q[1] or (np.isnan(p[1]) and np.isnan(q[1])))
-            assert [v[2] for v in a.viewpoints_] == sorted((v[2] for v in a.viewpoints_), reverse=True)
+        for key, v in mirror_arrays("f%d_visit_" % k, mine.frontiers_).items():
+            P.check(key, v)
+        for key, v in mirror_arrays("f%d_dormant_" % k, mine.dormant_frontiers_).items():
+            P.check(key, v)
+        P.check("f%d_ids" % k, [a.id_ for a in mine.frontiers_])
+        for i, a in enumerate(mine.frontiers_):
+            vp = a.viewpoints_
+            P.check("f%d_vp%d" % (k, i), viewpoint_rows([v[2] for v in vp], [v[1] for v in vp], [v[0] for v in vp]))
+            assert [v[2] for v in vp] == sorted((v[2] for v in vp), reverse=True)
     assert total_removed >= 3 and len(mine.frontiers_) >= 2   # the episode did exercise removal and survival
-    rff.close()
-    ref.close()
+
+
+REF_PINS = {"episode": (ref_episode, [()])}

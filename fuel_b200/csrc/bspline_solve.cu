@@ -401,6 +401,9 @@ __global__ void __launch_bounds__(WPB * 32) optimize_gram_kernel(
       }
       break;
     }
+    // with no stored pair the direction is steepest descent, -pg (the scale of the last pair does not carry over a
+    // restart: a failed line search or a non-descent direction empties the history)
+    if (cnt == 0) gamma = 1.f;
     // ---- two-loop recursion on fp32 scalars (every lane the same values; Gram data by broadcast reads).  The Gram
     // entries come out of an fp32 reduction, so fp32 arithmetic on them loses nothing; the result is only the search
     // direction -- acceptance (F, Armijo) and the iterate stay fp64.
@@ -580,6 +583,17 @@ __global__ void __launch_bounds__(WPB * 32) optimize_gram_kernel(
       if (lane == 1) YYg[head * M + head] = yy;
       if (lane == 4) Ug[head] = mine;
       if (lane == 5) Wg[head] = mine;
+    }
+    if (!keep && cnt == m) {
+      // the refused pair leaves the full ring as it is, so the oldest pair (slot head) stays in use -- and the batch
+      // above skipped it as the pair about to be dropped: bring its s.pg, y.pg up to date here (warp-uniform, rare)
+      const float4 s4 = S4[head * 32 + lane], y4 = Y4[head * 32 + lane];
+      const float st[3] = {s4.x, s4.y, s4.z}, yt[3] = {y4.x, y4.y, y4.z};
+      const float u = (float)wsum_x(f3(st, pgf)), wv = (float)wsum_x(f3(yt, pgf));
+      if (lane == 0) {
+        Ug[head] = u;
+        Wg[head] = wv;
+      }
     }
     if (keep) {
       S4[head * 32 + lane] = make_float4(sf[0], sf[1], sf[2], 0.f);

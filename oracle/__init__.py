@@ -87,7 +87,16 @@ class OrcTrajConst(C.Structure):
 
 
 class OrcSolveParams(C.Structure):
-    _fields_ = [("max_eval", C.c_int32), ("lbfgs_m", C.c_int32), ("xtol_rel", C.c_double)]
+    _fields_ = [("max_eval", C.c_int32), ("lbfgs_m", C.c_int32), ("xtol_rel", C.c_double), ("flags", C.c_int32),
+                ("reserved", C.c_int32)]
+
+
+class OrcSolveTrace(C.Structure):
+    _fields_ = [(k, C.c_int32) for k in ("n_kept", "n_curv_reject", "n_full_reject", "n_restart", "n_ls_fail",
+                                          "first_full_reject", "first_ls_fail")]
+
+
+SOLVE_EXACT_EVALS = 1
 
 
 _lib = None
@@ -656,15 +665,29 @@ def combine_cost_batch(g, dist_buf, p, tcs, n_pts, mask, x, threads=1):
     return f, grad
 
 
-def optimize_batch(g, dist_buf, p, tcs, n_pts, mask, x, max_eval=64, lbfgs_m=6, xtol_rel=1e-5, threads=1):
-    """CPU twin of fuelgpu_bspline_optimize_batch (NOT NLopt).  Returns (x_best, f_best, n_eval)."""
+def optimize_batch(g, dist_buf, p, tcs, n_pts, mask, x, max_eval=64, lbfgs_m=6, xtol_rel=1e-5, threads=1,
+                   exact_evals=False, trace=False):
+    """CPU twin of fuelgpu_bspline_optimize_batch (NOT NLopt).  Returns (x_best, f_best, n_eval).
+    exact_evals: the FUELGPU_SOLVE_EXACT_EVALS mode (max_eval evaluations, restarts instead of stops).
+    trace=True appends a dict of per-trajectory arrays: the OrcSolveTrace fields ([B] each) and "margin"
+    [B][max_eval], the smallest relative margin of the branch decisions taken up to each evaluation count."""
     x = np.array(x, dtype=np.float64, order="C", copy=True)
     B = x.shape[0]
     dist_buf = np.ascontiguousarray(dist_buf, dtype=np.float64)
     sp = OrcSolveParams()
     sp.max_eval, sp.lbfgs_m, sp.xtol_rel = max_eval, lbfgs_m, xtol_rel
+    sp.flags = SOLVE_EXACT_EVALS if exact_evals else 0
     fb = np.empty(B, dtype=np.float64)
     ne = np.empty(B, dtype=np.int32)
-    lib().orc_optimize_batch(C.byref(g), _p(dist_buf), C.byref(p), tcs, C.c_int32(n_pts), C.c_int32(mask),
-                             C.c_int32(B), C.byref(sp), _p(x), _p(fb), _p(ne), C.c_int(threads))
-    return x, fb, ne
+    args = (C.byref(g), _p(dist_buf), C.byref(p), tcs, C.c_int32(n_pts), C.c_int32(mask), C.c_int32(B), C.byref(sp),
+            _p(x), _p(fb), _p(ne))
+    if not trace:
+        lib().orc_optimize_batch(*args, C.c_int(threads))
+        return x, fb, ne
+    tr = (OrcSolveTrace * B)()
+    margin = np.empty((B, max_eval), dtype=np.float64)
+    lib().orc_optimize_batch_traced(*args, tr, _p(margin), C.c_int(threads))
+    t = np.frombuffer(tr, dtype=np.int32).reshape(B, len(OrcSolveTrace._fields_))
+    out = {name: t[:, i].copy() for i, (name, _) in enumerate(OrcSolveTrace._fields_)}
+    out["margin"] = margin
+    return x, fb, ne, out

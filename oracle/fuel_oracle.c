@@ -1185,17 +1185,32 @@ static double vdot(const double* a, const double* b, int n) {
   return s;
 }
 
+/* relative margin of a decision "a OP b": how far apart the two sides are, over the scale of either */
+static double rel_margin(double a, double b, double scale) {
+  const double m = fabs(a - b) / scale;
+  return m == m ? m : 0.0;  /* NaN (0/0, inf-inf): no margin */
+}
+
 static void optimize_one(const OrcGrid* g, const double* dist_buf, const OrcOptParams* p,
                          const OrcTrajConst* tc, int n, int mask, const OrcSolveParams* sp, double* x,
-                         double* f_best, int32_t* n_eval) {
+                         double* f_best, int32_t* n_eval, OrcSolveTrace* tr, double* mg) {
   const int opt_time = (mask & ORC_MINTIME) != 0;
   const int nv = opt_time ? 3 * n + 1 : 3 * n;
   const int m = sp->lbfgs_m;
+  const int exact = (sp->flags & ORC_SOLVE_EXACT_EVALS) != 0;
   double X[ORC_MAXVAR], G[ORC_MAXVAR], lb[ORC_MAXVAR], ub[ORC_MAXVAR], PG[ORC_MAXVAR], D[ORC_MAXVAR],
       Q[ORC_MAXVAR], XN[ORC_MAXVAR], GN[ORC_MAXVAR], dx[ORC_MAXVAR];
   static _Thread_local double S[ORC_MAXM][ORC_MAXVAR], Y[ORC_MAXM][ORC_MAXVAR];
   double rho[ORC_MAXM] = { 0 }, alpha[ORC_MAXM];
   int act[ORC_MAXVAR];
+  /* trace: mcur = smallest decision margin so far; it is written to mg[k-1] when the count leaves k */
+  double mcur = INFINITY;
+  OrcSolveTrace tdummy;
+  if (!tr) tr = &tdummy;
+  memset(tr, 0, sizeof(*tr));
+  tr->first_full_reject = tr->first_ls_fail = -1;
+#define NOTE(v) do { const double v_ = (v); if (!(v_ >= mcur)) mcur = v_ == v_ ? v_ : 0.0; } while (0)
+#define BUMP() do { if (mg) mg[neval - 1] = mcur; ++neval; } while (0)
   for (int i = 0; i < 3 * n; ++i) {
     const int k = i % 3;
     const double bmin = g->box_mind[k] + 0.1, bmax = g->box_maxd[k] - 0.1;
@@ -1224,7 +1239,15 @@ static void optimize_one(const OrcGrid* g, const double* dist_buf, const OrcOptP
       PG[i] = act[i] ? 0.0 : G[i];
     }
     const double pgn2 = vdot(PG, PG, nv);
-    if (!(pgn2 > 1e-24)) break;
+    NOTE(rel_margin(pgn2, 1e-24, fmax(pgn2, 1e-24)));
+    if (!(pgn2 > 1e-24)) {
+      if (!exact) break;
+      while (neval < sp->max_eval) { /* nothing left to descend: evaluate in place */
+        orc_combine_cost(g, dist_buf, p, tc, n, mask, X, &F, G);
+        BUMP();
+      }
+      break;
+    }
     memcpy(Q, PG, sizeof(double) * nv);
     for (int j = 0; j < cnt; ++j) {
       const int slot = (head - 1 - j + 2 * ORC_MAXM * m) % m;
@@ -1243,17 +1266,20 @@ static void optimize_one(const OrcGrid* g, const double* dist_buf, const OrcOptP
     }
     for (int i = 0; i < nv; ++i) D[i] = act[i] ? 0.0 : -Q[i];
     double gd = vdot(G, D, nv);
+    NOTE(rel_margin(gd, 0.0, sqrt(vdot(G, G, nv) * vdot(D, D, nv))));
     if (!(gd < 0.0)) {
       for (int i = 0; i < nv; ++i) D[i] = -PG[i];
       gd = -pgn2;
       cnt = 0;
+      ++tr->n_restart;
     }
     double step = cnt == 0 ? fmin(1.0, 1.0 / sqrt(pgn2)) : 1.0;
     int accepted = 0;
     while (neval < sp->max_eval) {
       for (int i = 0; i < nv; ++i) XN[i] = fmax(fmin(X[i] + step * D[i], ub[i]), lb[i]);
       orc_combine_cost(g, dist_buf, p, tc, n, mask, XN, &FN, GN);
-      ++neval;
+      BUMP();
+      NOTE(rel_margin(FN, best, fmax(fabs(FN), fabs(best))));
       if (FN < best) {
         best = FN;
         memcpy(x, XN, sizeof(double) * nv);
@@ -1261,6 +1287,7 @@ static void optimize_one(const OrcGrid* g, const double* dist_buf, const OrcOptP
       }
       for (int i = 0; i < nv; ++i) dx[i] = XN[i] - X[i];
       const double dec = vdot(G, dx, nv);
+      NOTE(rel_margin(FN, F + 1e-4 * dec, fmax(fabs(FN), fabs(F))));
       if (FN <= F + 1e-4 * dec) {
         accepted = 1;
         break;
@@ -1268,28 +1295,67 @@ static void optimize_one(const OrcGrid* g, const double* dist_buf, const OrcOptP
       step *= 0.5;
       if (step < 1e-12) break;
     }
-    if (!accepted) break;
+    if (!accepted) {
+      if (neval < sp->max_eval) { /* (a search cut short by the budget is not a failure) */
+        ++tr->n_ls_fail;
+        if (tr->first_ls_fail < 0) tr->first_ls_fail = neval;
+      }
+      if (!exact) break;
+      cnt = 0;
+      continue;
+    }
     int small = 1;
+    double xmargin = INFINITY, xfail = 0.0; /* xtol: the tightest component if all pass, the clearest failure if not */
     double s_[ORC_MAXVAR], y_[ORC_MAXVAR];
     for (int i = 0; i < nv; ++i) {
       s_[i] = XN[i] - X[i];
       y_[i] = GN[i] - G[i];
-      small = small && (fabs(s_[i]) <= sp->xtol_rel * fabs(XN[i]));
+      const double lim = sp->xtol_rel * fabs(XN[i]);
+      const int ok = fabs(s_[i]) <= lim;
+      small = small && ok;
+      const double mi = rel_margin(fabs(s_[i]), lim, fmax(fabs(s_[i]), lim));
+      if (ok) xmargin = fmin(xmargin, mi);
+      else xfail = fmax(xfail, mi);
     }
+    if (!exact) NOTE(small ? xmargin : xfail);
     const double sy = vdot(s_, y_, nv), ss = vdot(s_, s_, nv), yy = vdot(y_, y_, nv);
+    NOTE(rel_margin(sy, 1e-10 * sqrt(ss * yy), sqrt(ss * yy)));
     if (sy > 1e-10 * sqrt(ss * yy)) {
       memcpy(S[head], s_, sizeof(double) * nv);
       memcpy(Y[head], y_, sizeof(double) * nv);
       rho[head] = 1.0 / sy;
       head = (head + 1) % m;
       if (cnt < m) ++cnt;
+      ++tr->n_kept;
+    } else {
+      ++tr->n_curv_reject;
+      if (cnt == m) {
+        ++tr->n_full_reject;
+        if (tr->first_full_reject < 0) tr->first_full_reject = neval;
+      }
     }
     memcpy(X, XN, sizeof(double) * nv);
     memcpy(G, GN, sizeof(double) * nv);
     F = FN;
-    if (small) break;
+    if (!exact && small) break;
   }
   *n_eval = neval;
+  if (mg)
+    for (int k = neval; k <= sp->max_eval; ++k) mg[k - 1] = mcur;
+#undef NOTE
+#undef BUMP
+}
+
+void orc_optimize_batch_traced(const OrcGrid* g, const double* dist_buf, const OrcOptParams* p,
+                               const OrcTrajConst* tc, int32_t n_pts, int32_t cost_mask, int32_t B,
+                               const OrcSolveParams* sp, double* x, double* f_best, int32_t* n_eval,
+                               OrcSolveTrace* trace, double* margin, int threads) {
+  const int nv = (cost_mask & ORC_MINTIME) ? 3 * n_pts + 1 : 3 * n_pts;
+  if (threads < 1) threads = 1;
+#pragma omp parallel for num_threads(threads) schedule(dynamic, 8)
+  for (int b = 0; b < B; ++b)
+    optimize_one(g, dist_buf, p, &tc[b], n_pts, cost_mask, sp, x + (int64_t)b * nv, &f_best[b], &n_eval[b],
+                 trace ? &trace[b] : NULL, margin ? margin + (int64_t)b * sp->max_eval : NULL);
 }
 
 void orc_optimize_batch(const OrcGrid* g, const double* dist_buf, const OrcOptParams* p,
@@ -1300,5 +1366,6 @@ void orc_optimize_batch(const OrcGrid* g, const double* dist_buf, const OrcOptPa
   if (threads < 1) threads = 1;
 #pragma omp parallel for num_threads(threads) schedule(dynamic, 8)
   for (int b = 0; b < B; ++b)
-    optimize_one(g, dist_buf, p, &tc[b], n_pts, cost_mask, sp, x + (int64_t)b * nv, &f_best[b], &n_eval[b]);
+    optimize_one(g, dist_buf, p, &tc[b], n_pts, cost_mask, sp, x + (int64_t)b * nv, &f_best[b], &n_eval[b], NULL,
+                 NULL);
 }

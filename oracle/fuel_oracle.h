@@ -229,11 +229,37 @@ typedef struct {
   int32_t max_eval;   /* max_iteration_num_[id] */
   int32_t lbfgs_m;    /* history length */
   double xtol_rel;    /* 1e-5, :173 */
+  int32_t flags;      /* ORC_SOLVE_* (same bits as FUELGPU_SOLVE_*) */
+  int32_t reserved;
 } OrcSolveParams;
+/* FUELGPU_SOLVE_EXACT_EVALS: a vanished projected gradient re-evaluates in place until max_eval, a failed line
+ * search drops the history and goes on from steepest descent, and there is no xtol stop */
+#define ORC_SOLVE_EXACT_EVALS 1
 void orc_optimize_batch(const OrcGrid* g, const double* dist_buf, const OrcOptParams* p,
                         const OrcTrajConst* tc, int32_t n_pts, int32_t cost_mask, int32_t B,
                         const OrcSolveParams* sp, double* x /*[B][nvar] in/out*/,
                         double* f_best /*[B]*/, int32_t* n_eval /*[B]*/, int threads);
+
+/* What the solver decided for one trajectory: event counts, and when the first of the two rare events happened
+ * (the evaluation count at that moment; -1: never). */
+typedef struct {
+  int32_t n_kept;          /* (s, y) pairs stored */
+  int32_t n_curv_reject;   /* pairs refused by the curvature test */
+  int32_t n_full_reject;   /* ... of them while the history ring was full */
+  int32_t n_restart;       /* non-descent directions replaced by steepest descent */
+  int32_t n_ls_fail;       /* line searches that ended without an Armijo step */
+  int32_t first_full_reject;
+  int32_t first_ls_fail;
+} OrcSolveTrace;
+/* orc_optimize_batch with a decision trace (either output may be NULL; results are bit for bit those of
+ * orc_optimize_batch).  margin [B][max_eval]: entry k-1 is the smallest relative margin of every branch decision
+ * taken while the evaluation count was <= k -- pgn2 > 1e-24, g.d < 0, f < best, the Armijo test, the curvature
+ * test and the xtol test -- so a solver that rounds differently takes the same path through its first k
+ * evaluations whenever its disagreement stays below that margin. */
+void orc_optimize_batch_traced(const OrcGrid* g, const double* dist_buf, const OrcOptParams* p,
+                               const OrcTrajConst* tc, int32_t n_pts, int32_t cost_mask, int32_t B,
+                               const OrcSolveParams* sp, double* x, double* f_best, int32_t* n_eval,
+                               OrcSolveTrace* trace /*[B]*/, double* margin /*[B][max_eval]*/, int threads);
 
 #ifdef __cplusplus
 }

@@ -82,11 +82,36 @@ def test_benchmark_objective(fuel, orc, scene):
     assert np.array_equal(f, f2) and np.array_equal(g, g2)
 
 
+# control-point counts: 7, 8, 31, 32 run the warp kernels (one lane per point; 7 has a single interior segment,
+# 32 fills the warp), 33 .. 64 the thread kernel, which only the faithful evaluator has
+N_WARP = [7, 8, 20, 31, 32]
+N_THREAD = [33, 47, 64]
+
+
+def trajectories(scene, B, n, seed):
+    # lines longer than the 0.35 m spacing allows inside the 18 m x 10 m box would never be drawn
+    return W.make_trajectories(scene["g"], scene["inflate"], B=B, n_pts=n, seed=seed, spacing=0.35 if n <= 32 else 0.2)
+
+
+def check_both(fuel, opt, x, tg, n, mask, fr, gr):
+    """the faithful evaluator (both kernels) and, where it exists (n <= 32), the solver's fast one"""
+    f, g = opt.combineCostBatch(x, tg, n, mask)
+    check(f, g, fr, gr)
+    if n <= 32:
+        f, g = opt.combineCostBatch(x, tg, n, mask, fast_eval=True)
+        check(f, g, fr, gr)
+    else:
+        with pytest.raises(fuel.FuelGpuError) as e:
+            opt.combineCostBatch(x, tg, n, mask, fast_eval=True)
+        assert e.value.code == fuel._lib.EUNSUPPORTED
+
+
+@pytest.mark.parametrize("n_pts", N_WARP + N_THREAD)
 @pytest.mark.parametrize("mask_name", ["SMOOTHNESS", "DISTANCE", "FEASIBILITY", "START", "END", "MINTIME",
                                        "NORMAL_PHASE"])
-def test_single_terms(fuel, orc, scene, mask_name):
-    B, N = 64, 20
-    tr = W.make_trajectories(scene["g"], scene["inflate"], B=B, n_pts=N, seed=5)
+def test_single_terms(fuel, orc, scene, mask_name, n_pts):
+    B, N = 64, n_pts
+    tr = trajectories(scene, B, N, seed=5)
     O = fuel.BsplineOptimizer
     mask = getattr(O, mask_name)
     if mask_name == "MINTIME":
@@ -97,24 +122,36 @@ def test_single_terms(fuel, orc, scene, mask_name):
         x[::2, -1] *= 0.5
     else:
         tr["dt"][::2] *= 0.5
-    f, g = scene["opt"].combineCostBatch(x, gpu_consts(fuel, tr, B), N, mask)
     fr, gr = orc.combine_cost_batch(orc_grid(orc, scene["g"]), scene["d64"], orc.opt_params(),
                                     orc_consts(orc, tr, B), N, mask, x)
-    check(f, g, fr, gr)
+    check_both(fuel, scene["opt"], x, gpu_consts(fuel, tr, B), N, mask, fr, gr)
 
 
 def test_guide_waypoints_end3_timelb(fuel, orc, scene):
-    """GUIDE_PHASE, WAYPOINTS, a 3-entry end_state_ and an active time lower bound."""
-    B, N = 32, 24
-    tr = W.make_trajectories(scene["g"], scene["inflate"], B=B, n_pts=N, seed=9)
+    """GUIDE_PHASE, WAYPOINTS (one at the last legal index, idx + 2 == N - 1), a 3-entry end_state_ and an active
+    time lower bound, at 24 control points."""
+    guide_waypoints_end3_timelb(fuel, orc, scene, 24)
+
+
+@pytest.mark.parametrize("n_pts", [7, 8, 31, 32] + N_THREAD)
+def test_guide_waypoints_end3_timelb_n_pts(fuel, orc, scene, n_pts):
+    """The same at the warp kernels' edges and on the thread kernel."""
+    guide_waypoints_end3_timelb(fuel, orc, scene, n_pts)
+
+
+def guide_waypoints_end3_timelb(fuel, orc, scene, n_pts):
+    B, N = 32, n_pts
+    tr = trajectories(scene, B, N, seed=9)
     O = fuel.BsplineOptimizer
     rng = np.random.default_rng(3)
     guide = tr["ctrl"][:, 3:N - 3] + rng.normal(scale=0.2, size=(B, N - 6, 3))
-    widx = [0, 4, 9, N - 3]
-    waypt = rng.uniform(-1, 1, size=(B, len(widx), 3)) + tr["ctrl"][:, [1, 5, 10, N - 2]]
+    widx = sorted({i for i in (0, 4, 9) if i < N - 3} | {N - 3})
+    waypt = rng.uniform(-1, 1, size=(B, len(widx), 3)) + tr["ctrl"][:, [i + 1 for i in widx]]
     time_lb = (N - 3) * tr["dt"] * 1.3
     for mask, n_end in ((O.GUIDE_PHASE, 1), (O.SMOOTHNESS | O.WAYPOINTS, 1), (O.NORMAL_PHASE | O.MINTIME, 3),
                         (O.SMOOTHNESS | O.WAYPOINTS | O.START | O.END, 2)):
+        if N + int(bool(mask & O.MINTIME)) > 64:
+            continue
         x = W.pack_x(tr["ctrl"], tr["dt"], mintime=bool(mask & O.MINTIME))
         kw = dict(guide=guide, waypt=waypt, waypt_idx=widx, n_end=n_end, time_lb=time_lb)
         tg = gpu_consts(fuel, tr, B, **kw)
@@ -126,9 +163,8 @@ def test_guide_waypoints_end3_timelb(fuel, orc, scene):
                         v = float(rng.normal())
                         tg[b].end[i][k] = v
                         to[b].end[i][k] = v
-        f, g = scene["opt"].combineCostBatch(x, tg, N, mask)
         fr, gr = orc.combine_cost_batch(orc_grid(orc, scene["g"]), scene["d64"], orc.opt_params(), to, N, mask, x)
-        check(f, g, fr, gr)
+        check_both(fuel, scene["opt"], x, tg, N, mask, fr, gr)
 
 
 def test_adversarial_positions(fuel, orc, scene):
@@ -259,27 +295,42 @@ def test_fast_evaluator_is_what_the_parity_bar_covers(fuel, orc, scene):
         check(f, gg, fr, gr)
         f2, g2 = scene["opt"].combineCostBatch(x, gpu_consts(fuel, tr, B), 20, mask)
         assert not (np.array_equal(f, f2) and np.array_equal(gg, g2)), "the flag did not switch evaluators"
+    fast_evaluator_adversarial_and_single_terms(fuel, orc, scene, 20)
+
+
+@pytest.mark.parametrize("n_pts", [7, 8, 31, 32])
+def test_fast_evaluator_n_pts(fuel, orc, scene, n_pts):
+    """The fast evaluator's adversarial positions and single terms at the edges of its warp layout (one lane per
+    control point: a single interior segment at 7, a full warp at 32)."""
+    fast_evaluator_adversarial_and_single_terms(fuel, orc, scene, n_pts)
+
+
+def fast_evaluator_adversarial_and_single_terms(fuel, orc, scene, n_pts):
+    O = fuel.BsplineOptimizer
+    g = scene["g"]
+    og = orc_grid(orc, g)
+    mask = O.NORMAL_PHASE | O.MINTIME
     # adversarial positions: map boundary, outside the map, the isInMap margin
     B = 48
-    tr = W.make_trajectories(g, scene["inflate"], B=B, n_pts=20, seed=13)
+    tr = W.make_trajectories(g, scene["inflate"], B=B, n_pts=n_pts, seed=13)
     ctrl = tr["ctrl"].copy()
-    ctrl[0:8, 5] = g.origin + [0.02, 0.5, 0.5]
-    ctrl[8:16, 7] = g.map_max + 0.3
-    ctrl[16:24, 9] = g.map_max - [1e-4, 0.5, 0.5]
+    ctrl[0:8, 5 * n_pts // 20] = g.origin + [0.02, 0.5, 0.5]
+    ctrl[8:16, 7 * n_pts // 20] = g.map_max + 0.3
+    ctrl[16:24, 9 * n_pts // 20] = g.map_max - [1e-4, 0.5, 0.5]
     tr["ctrl"] = ctrl
     x = W.pack_x(ctrl, tr["dt"])
-    f, gg = scene["opt"].combineCostBatch(x, gpu_consts(fuel, tr, B), 20, mask, fast_eval=True)
-    fr, gr = orc.combine_cost_batch(og, scene["d64"], orc.opt_params(), orc_consts(orc, tr, B), 20, mask, x)
+    f, gg = scene["opt"].combineCostBatch(x, gpu_consts(fuel, tr, B), n_pts, mask, fast_eval=True)
+    fr, gr = orc.combine_cost_batch(og, scene["d64"], orc.opt_params(), orc_consts(orc, tr, B), n_pts, mask, x)
     check(f, gg, fr, gr)
     # every single term through the fast evaluator
-    tr = W.make_trajectories(g, scene["inflate"], B=64, n_pts=20, seed=5)
+    tr = W.make_trajectories(g, scene["inflate"], B=64, n_pts=n_pts, seed=5)
     for name in ("SMOOTHNESS", "DISTANCE", "FEASIBILITY", "START", "END"):
         m1 = getattr(O, name)
         x = W.pack_x(tr["ctrl"], tr["dt"] * 0.6, mintime=False)
         tr2 = dict(tr)
         tr2["dt"] = tr["dt"] * 0.6
-        f, gg = scene["opt"].combineCostBatch(x, gpu_consts(fuel, tr2, 64), 20, m1, fast_eval=True)
-        fr, gr = orc.combine_cost_batch(og, scene["d64"], orc.opt_params(), orc_consts(orc, tr2, 64), 20, m1, x)
+        f, gg = scene["opt"].combineCostBatch(x, gpu_consts(fuel, tr2, 64), n_pts, m1, fast_eval=True)
+        fr, gr = orc.combine_cost_batch(og, scene["d64"], orc.opt_params(), orc_consts(orc, tr2, 64), n_pts, m1, x)
         check(f, gg, fr, gr)
 
 

@@ -240,7 +240,8 @@ __device__ __forceinline__ int unpack_v(uint32_t e) { return (int)(e >> 22); }
 __device__ __forceinline__ int unpack_h(uint32_t e) { return (int)(e & 0x3fffffu); }
 __device__ __forceinline__ float fast_sqrt(float x) {
   float r;
-  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));  // <= 1 ulp-ish; the bar is 1e-4 relative
+  // a few units of 2^-24: rint((dist/res)^2) still gives back the exact integer d2 up to 2^20 (tests/helpers.py)
+  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
   return r;
 }
 

@@ -50,6 +50,78 @@ def orc_grid(orc, g):
     return orc.make_grid(g.n, g.res, g.origin, g.box_min, g.box_max)
 
 
+ESDF_SENTINEL = 1e150  # the reference holds resolution*sqrt(DBL_MAX) ~ 1.34e153 where the box has no site
+EXACT_N_MAX = 1 << 20
+# largest |(got/res)^2 - N_ref| assert_esdf_exact has seen in this process (N_ref <= EXACT_N_MAX)
+ESDF_EXACT_STATS = {"max_dev": 0.0, "voxels": 0}
+
+
+def _esdf_box(got, ref, box):
+    if box is None:
+        return got, ref
+    sl = tuple(slice(int(box[0][i]), int(box[1][i]) + 1) for i in range(3))
+    return got[sl], ref[sl]
+
+
+def _esdf_sentinel(got, ref):
+    """+inf on the device exactly where the reference holds its sentinel, with the same sign (a signed field whose box
+    is all inflated ends at -inf); returns the mask of finite reference values"""
+    nosite = np.abs(ref) > ESDF_SENTINEL
+    assert np.array_equal(np.isinf(got), nosite), "sentinel mismatch at %d voxels" % int(
+        np.count_nonzero(np.isinf(got) != nosite))
+    assert np.array_equal(np.signbit(got[nosite]), np.signbit(ref[nosite])), "sentinel sign mismatch"
+    return ~nosite
+
+
+def assert_esdf_rel(got_f32, ref_f64, box=None, rtol=1e-4):
+    """The relative bar: |got - ref| <= rtol*|ref| where the reference is finite, plus the sentinel check."""
+    got, ref = _esdf_box(got_f32, ref_f64, box)
+    fin = _esdf_sentinel(got, ref)
+    g, r = got[fin].astype(np.float64), ref[fin]
+    err = np.abs(g - r)
+    assert np.all(err <= rtol * np.abs(r)), "max rel err %g" % np.max(err / np.maximum(np.abs(r), 1e-12))
+
+
+def assert_esdf_exact(got_f32, ref_f64, res, box=None, signed=False):
+    """The device field against the fp64 reference to the exact squared voxel distance N.
+
+    Every finite intermediate of the transform is an integer N, and the device stores fl32(res32 * sqrt.approx(N))
+    (res32 = float32(res)): a relative error of a few units of 2^-24, so (got/res32)^2 is within 0.4 of N up to
+    N = 2^20, while N +- 1 moves the distance by only ~1/(2N) relative (5e-5 at N = 10^4, below a 1e-4 relative bar).
+    So N_dev = rint((got/res32)^2) must equal N_ref = rint((ref/res)^2) wherever N_ref <= 2^20, and the largest
+    |(got/res32)^2 - N_ref| must stay below 0.45; above 2^20 (diagonals over 1024 voxels) the 1e-4 relative bar
+    applies.  Signed fields (esdf.cu signed_merge_kernel: dist += res - neg where neg > 0) are recovered from d where
+    the reference is positive and from res - d where it is <= 0.  Returns the largest deviation."""
+    got, ref = _esdf_box(got_f32, ref_f64, box)
+    fin = _esdf_sentinel(got, ref)
+    g, r = got[fin].astype(np.float64), ref[fin]
+    res32 = float(np.float32(res))
+    if signed:
+        neg = r <= 0.0
+        g = np.where(neg, res32 - g, g)
+        r = np.where(neg, res - r, r)
+    q_ref = (r / res) ** 2
+    n_ref = np.rint(q_ref)
+    assert np.all(np.abs(q_ref - n_ref) < 1e-6), "the reference is not res*sqrt(integer)"
+    q_dev = (g / res32) ** 2
+    small = n_ref <= EXACT_N_MAX
+    dev = np.abs(q_dev[small] - n_ref[small])
+    worst = float(dev.max()) if dev.size else 0.0
+    bad = np.count_nonzero(np.rint(q_dev[small]) != n_ref[small])
+    if bad:
+        i = int(np.argmax(dev))
+        raise AssertionError("squared voxel distance differs at %d of %d voxels (e.g. N_dev %.3f vs N_ref %d)" %
+                             (bad, dev.size, q_dev[small][i], n_ref[small][i]))
+    assert worst < 0.45, "largest |(got/res)^2 - N| %.3f: the device rounding is worse than its derivation" % worst
+    big = ~small
+    if np.any(big):
+        gb, rb = got[fin][big].astype(np.float64), ref[fin][big]
+        assert np.all(np.abs(gb - rb) <= 1e-4 * np.abs(rb)), "relative error above 1e-4 beyond N = 2^20"
+    ESDF_EXACT_STATS["max_dev"] = max(ESDF_EXACT_STATS["max_dev"], worst)
+    ESDF_EXACT_STATS["voxels"] += int(dev.size)
+    return worst
+
+
 def rel_err(a, b, floor=0.0):
     a = np.asarray(a, dtype=np.float64)
     b = np.asarray(b, dtype=np.float64)

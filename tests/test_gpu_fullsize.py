@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 from fuel_b200 import workloads as W
-from tests.helpers import make_sdf_map, orc_grid
+from tests.helpers import assert_esdf_exact, make_sdf_map, orc_grid
 
 pytestmark = pytest.mark.gpu
 
@@ -44,9 +44,7 @@ def test_esdf_512_slab_matches_oracle(fuel, orc, pillar):
     m.updateESDF3d()
     d = m.download()[:, :, 200:224].copy()
     ref = orc.update_esdf3d(orc_grid(orc, g), inflate, tri, bmin, bmax, True, False, threads=16)[:, :, 200:224]
-    fin = ref < 1e150
-    assert np.array_equal(np.isinf(d), ~fin)
-    assert np.all(np.abs(d[fin] - ref[fin]) <= 1e-4 * ref[fin])
+    assert_esdf_exact(d, ref, g.res)
     m.local_bound_min_, m.local_bound_max_ = np.zeros(3, dtype=np.int32), np.array(g.n) - 1
 
 
@@ -61,10 +59,7 @@ def test_esdf_512_full_box_matches_oracle(fuel, orc, variant):
     d = m.download().copy()
     m.close()
     ref = orc.update_esdf3d(orc_grid(orc, g), inflate, tri, [0, 0, 0], np.array(g.n) - 1, True, False, threads=16)
-    fin = ref < 1e150
-    assert np.array_equal(np.isinf(d), ~fin)
-    err = np.abs(d[fin].astype(np.float64) - ref[fin])
-    assert np.all(err <= 1e-4 * ref[fin]), float(np.max(err / np.maximum(ref[fin], 1e-12)))
+    assert_esdf_exact(d, ref, g.res)
     del ref
 
 
